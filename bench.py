@@ -82,7 +82,13 @@ def parse():
     p.add_argument("--breakdown-iters", type=int, default=6)
     p.add_argument("--p", type=float, default=0.5, help="config c3: node2vec return parameter")
     p.add_argument("--q", type=float, default=2.0, help="config c3: node2vec in-out parameter")
+    p.add_argument("--dump-outputs", metavar="DIR", default=None,
+                   help="after the timed steps, write what the last timed step returned to DIR/<name>.npy (float32 / float64, "
+                        "at most 64 MB in all; arrays too large for that keep a fixed seeded sample of their rows)")
     a = p.parse_args()
+    if a.dump_outputs and (a.impl != "ours" or a.config in ("c3", "c5") or int(os.environ.get("WORLD_SIZE", "1")) > 1
+                           or os.environ.get("EU_BENCH_FORCE_SHARDED")):
+        p.error("--dump-outputs covers the single-GPU minibatch step (--impl ours, config c4 or c2, one rank)")
     cfg = CONFIGS[a.config]
     for k in ("nodes", "edges", "batch", "fanout", "dim"):
         if getattr(a, k) is None:
@@ -195,6 +201,50 @@ class Clocks:
 
 
 # ----------------------------------------------------------------------------- our arm
+DUMP_BYTES = 63 * 10**6       # --dump-outputs payload; with the .npy headers the files stay under 64 MB
+
+
+def last_step_outputs(lane, counts):
+    """Host copies of what a caller of the step receives for the last batch of the lane's launch group: per hop the sampled
+    ids / weights / types, and per source hop the dense features and the neighbor means."""
+    b, G = lane.G - 1, lane.G
+    out = {}
+    for l in range(len(counts)):
+        per = lane.n[l + 1] // G
+        for name, xs in (("ids", lane.ids), ("weights", lane.w), ("types", lane.ty)):
+            out["%s_hop%d" % (name, l + 1)] = xs[l][b * per:(b + 1) * per].cpu().numpy()
+    for l in range(len(counts)):
+        per = lane.n[l] // G
+        out["features_hop%d" % l] = lane.x[l][b * per:(b + 1) * per].cpu().numpy()
+        out["neighbor_mean_hop%d" % l] = lane.agg[l][b * per:(b + 1) * per].cpu().numpy()
+    return out
+
+
+def dump_outputs(dirname, arrays):
+    """Writes DIR/<name>.npy per array: 64-bit integers as float64 (ids are exact below 2**53), everything else as float32.
+    Arrays are written whole, smallest first, while each fits an equal share of what is left of DUMP_BYTES; from the first that
+    does not, every remaining array gets an equal share as a sample of its rows -- the same rows on every run, and the same rows
+    for arrays of the same length -- whose indices go to DIR/<name>_rows.npy.  Returns {file: shape}."""
+    os.makedirs(dirname, exist_ok=True)
+    conv = {k: v.astype(np.float64 if v.dtype.kind in "iu" and v.dtype.itemsize > 4 else np.float32) for k, v in arrays.items()}
+    names = sorted(conv, key=lambda k: (conv[k].nbytes, k))
+    left, share, written = DUMP_BYTES, None, {}
+    for i, name in enumerate(names):
+        a = conv[name]
+        if share is None and a.nbytes > left // (len(names) - i):
+            share = left // (len(names) - i)
+        if share is not None:
+            k = share // (a[0].nbytes + 8)                      # + the row's float64 index
+            rows = np.sort(np.random.RandomState(0).permutation(len(a))[:k]).astype(np.float64)
+            np.save(os.path.join(dirname, name + "_rows.npy"), rows)
+            written[name + "_rows"] = rows.shape
+            a = a[rows.astype(np.int64)]
+        np.save(os.path.join(dirname, name + ".npy"), a)
+        written[name] = a.shape
+        left -= a.nbytes
+    return written
+
+
 def step_bytes(B, counts, D):
     """Algorithmic bytes (SURVEY.md section 8d).  Sampling: 48 B per sampled edge + 40 B per seed (CDF mode,
     mean degree 10).  Aggregation (fused): 8 B id + 4D B row read per edge, 4D B write per output row.
@@ -438,6 +488,7 @@ def run_ours(args):
     all_lanes = lanes + ([tail_lane] if tail_lane else [])
 
     host_lanes = []
+    last = {}                                            # the lane that ran the last step of the latest run()
 
     def run(n_steps, first, mode):
         """n_steps steps round-robin over the lanes; returns device ms (events on the main stream, lanes fork from / join
@@ -459,6 +510,8 @@ def run_ours(args):
             if use_tail and i == n_groups - 1:
                 ln, sd = tail_lane, sd[:rem * args.batch]
             work.append((ln, g0, sd))
+        if work:
+            last["lane"] = work[-1][0]
         torch.cuda.synchronize()
         ev0.record(main)
         for ln in all_lanes + host_lanes:
@@ -509,6 +562,9 @@ def run_ours(args):
     if use_graphs:
         launches = int(per_step_launches * args.steps)  # kernels of ours inside the replayed graphs
     clk = clocks.stop(w0, w1)
+    if args.dump_outputs:
+        files = dump_outputs(args.dump_outputs, last_step_outputs(last["lane"], counts))
+        print("--dump-outputs: %s" % ", ".join("%s.npy %s" % (k, v) for k, v in files.items()), file=sys.stderr)
     # end-to-end passes: warm EVERY lane the timed pass will use (a lane's first *_host call grows its pinned staging and device
     # scratch -- cudaHostAlloc / cudaMalloc of hundreds of MB, which one box in round 2 took 40 ms per step to do inside the timed
     # region), and the tail lane, before timing

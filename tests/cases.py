@@ -6,9 +6,10 @@ import os
 import numpy as np
 
 import graphs
-from golden.make_golden import NB_CASES, SYNTH  # noqa: F401
+from golden.make_golden import NB_CASES, SYNTH, digest  # noqa: F401
 
 _G = None
+_REF = None
 
 
 def golden():
@@ -16,6 +17,21 @@ def golden():
     if _G is None:
         _G = np.load(os.path.join(graphs.GOLDEN, "golden_ops.npz"))
     return _G
+
+
+def ref_checks():
+    """tests/golden/ref_checks.npz: the reference's outputs (as digests) and the map orders of the random graphs"""
+    global _REF
+    if _REF is None:
+        z = np.load(os.path.join(graphs.GOLDEN, "ref_checks.npz"))
+        _REF = {k: z[k] for k in z.files}
+        _REF["digests"] = {k.decode(): v.tobytes() for k, v in zip(z["keys"], z["sha256"])}
+    return _REF
+
+
+def eq_ref(got, key, what):
+    """`got` is bit for bit what the reference returned for `key` (same shape, dtype and values; integers of any width)"""
+    assert digest(got) == ref_checks()["digests"][key], "%s: differs from the reference's output" % what
 
 
 def eq(a, b, what):
@@ -121,6 +137,9 @@ class OracleBackend:
 
     def sample_node(self, types, count):
         return self.og.sample_node(types, count, self._rng)
+
+    def sampler_tables(self, t):
+        return self.og.node_sampler_tables(t)
 
 
 class CudaBackend:

@@ -52,3 +52,41 @@ def test_cpu_arm_memory_cap():
     rows = a.batch * 15 * 10
     assert 1 <= cap <= bench.host_cores()
     assert cap * rows * a.dim * 4 * 2.6 <= 48 << 30    # the threads' minibatch buffers fit the budget
+
+
+def test_dump_outputs_are_the_last_batch_within_budget_and_repeat(tmp_path, monkeypatch):
+    """--dump-outputs: the last batch of the lane's launch group, as float32 / float64 files within the byte budget; arrays
+    that do not fit keep the same seeded rows on every run (and equal-length arrays the same rows)"""
+    import numpy as np
+    import torch
+    bench, _ = _parse([])
+    budget = 80_000
+    monkeypatch.setattr(bench, "DUMP_BYTES", budget)
+    B, counts, D, G = 64, [5, 4], 32, 3
+
+    class Lane:
+        pass
+    ln = Lane()
+    ln.G, ln.n = G, [G * B, G * B * 5, G * B * 20]
+    torch.manual_seed(0)
+    ln.ids = [torch.randint(-1, 10 ** 8, (n,), dtype=torch.int64) for n in ln.n[1:]]
+    ln.w = [torch.rand(n) for n in ln.n[1:]]
+    ln.ty = [torch.randint(0, 3, (n,), dtype=torch.int32) for n in ln.n[1:]]
+    ln.x = [torch.rand(ln.n[l], D) for l in range(2)]
+    ln.agg = [torch.rand(ln.n[l], D) for l in range(2)]
+    out = bench.last_step_outputs(ln, counts)
+    assert np.array_equal(out["ids_hop2"], ln.ids[1][-B * 20:].numpy())
+    assert np.array_equal(out["features_hop0"], ln.x[0][-B:].numpy())
+    assert np.array_equal(out["neighbor_mean_hop1"], ln.agg[1][-B * 5:].numpy())
+    a = bench.dump_outputs(str(tmp_path / "a"), out)
+    assert a == bench.dump_outputs(str(tmp_path / "b"), out)
+    total = 0
+    for name in a:
+        x = np.load(tmp_path / "a" / (name + ".npy"))
+        assert x.dtype in (np.float32, np.float64) and np.array_equal(x, np.load(tmp_path / "b" / (name + ".npy")))
+        total += x.nbytes
+    assert total <= budget
+    assert np.array_equal(np.load(tmp_path / "a" / "ids_hop2.npy").astype(np.int64), out["ids_hop2"])   # whole and exact
+    rows = np.load(tmp_path / "a" / "features_hop1_rows.npy")
+    assert 0 < len(rows) < B * 5 and np.array_equal(rows, np.load(tmp_path / "a" / "neighbor_mean_hop1_rows.npy"))
+    assert np.array_equal(np.load(tmp_path / "a" / "features_hop1.npy"), out["features_hop1"][rows.astype(np.int64)])

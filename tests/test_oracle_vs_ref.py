@@ -1,23 +1,20 @@
-"""CPU, where oracle/_ref/libeuler_ref.so exists: the C restatement against the UNMODIFIED reference
-sources on fresh random graphs (not only the committed golden cases)."""
+"""CPU: the C restatement against what the UNMODIFIED reference sources returned on fresh random graphs (not only the
+committed golden cases), stored by tests/golden/make_golden.py::write_ref_checks in tests/golden/ref_checks.npz."""
 import numpy as np
 import pytest
 
 import cases
 import graphs
+from golden import make_golden as mg
 from oracle import pyoracle as po
-
-pytestmark = pytest.mark.skipif(not po.have_ref(), reason="oracle/_ref not built (needs /root/reference)")
 
 
 def test_uniform_stream_bit_exact():
-    R = po.ref()
-    for s in (1, 12345, 0, 2147483647, 1758564000):
-        R.ref_seed(s)
-        r = po.Rng(s)
-        assert all(R.ref_uniform() == r.uniform() for _ in range(50000))
+    for s in mg.UNIFORM_SEEDS:
+        cases.eq_ref(mg.uniform_stream(po.Rng(s).uniform), "uniform%d" % s, "uniform stream of seed %d" % s)
 
 
+@pytest.mark.skipif(not po.have_ref(), reason="checks the reference's own loader: needs oracle/_ref (the reference sources at build time)")
 def test_reference_loader_reads_committed_fixture(tiny_dir):
     g = po.RefGraph.load(tiny_dir, "node", "node")
     csr = g.export_csr()
@@ -27,46 +24,19 @@ def test_reference_loader_reads_committed_fixture(tiny_dir):
     assert np.array_equal(g.node_ids_in_map_order(), z["map_order"])
 
 
-@pytest.mark.parametrize("seed,T,kw", [(1, 1, {}), (2, 2, dict(zero_w_frac=0.2)), (3, 4, dict(hub=300, id_stride=13)),
-                                       (4, 6, dict(empty_frac=0.5, n_node_types=3))])
+@pytest.mark.parametrize("seed,T,kw", mg.RANDOM_OPS)
 def test_random_graph_ops(seed, T, kw):
-    g = graphs.random_graph(seed=seed, n=400, T=T, avg_deg=5, **kw)
-    rg = graphs.ref_graph(g)
-    be = cases.OracleBackend(g, rg.node_ids_in_map_order())
-    rs = np.random.RandomState(seed)
-    seeds = g["ids"][rs.randint(0, 400, size=300)].astype(np.int64)
-    seeds[::9] = 12345678901
-    for et, cnt in [([0], 7), (list(range(T)), 20), ([T - 1, 0], 5), ([], 2), ([0, 0], 3)]:
-        rg.seed(seed); be.seed(seed)
-        for a, b in zip(rg.op_sample_neighbor(seeds, et, cnt, -7), be.op_sample_neighbor(seeds, et, cnt, -7)):
-            cases.eq(b, a, "sample_neighbor %s" % et)
-        assert rg.draws() == be.draws()
-    ets = [[0, T - 1], [0, T - 1], [T - 1, 0]]
-    rg.seed(seed + 1); be.seed(seed + 1)
-    a, b = rg.op_sample_fanout(seeds, ets, [4, 3, 2], -1), be.op_sample_fanout(seeds, ets, [4, 3, 2], -1)
-    for x, y in zip(a, b):
-        for l in range(3):
-            cases.eq(y[l], x[l], "fanout hop %d" % l)
-    wet = np.asarray([list(range(T))] * 10, np.int32)
-    for p, q in [(0.5, 2.0), (1.0, 1.0), (4.0, 0.25), (1.0, 2.0)]:
-        rg.seed(seed + 2); be.seed(seed + 2)
-        cases.eq(be.op_random_walk(seeds[:100], wet, p, q, -1), rg.op_random_walk(seeds[:100], wet, p, q, -1),
-                 "walk p=%s q=%s" % (p, q))
-    for types in ([-1], [0], list(range(g["n_node_types"]))):
-        rg.seed(seed + 3); be.seed(seed + 3)
-        cases.eq(be.sample_node(types, 300), rg.sample_node(types, 300), "sample_node %s" % types)
-    for t in range(g["n_node_types"]):
-        for x, y in zip(rg.sampler_tables(t), be.og.node_sampler_tables(t)):
-            cases.eq(y, x, "alias tables type %d" % t)
+    g = mg.random_ops_graph(seed, T, kw)
+    be = cases.OracleBackend(g, cases.ref_checks()["rops%d_map_order" % seed])
+    for k, x in mg.random_ops(be, g, seed).items():
+        cases.eq_ref(x, "rops%d_%s" % (seed, k), "graph %d: %s" % (seed, k))
 
 
 def test_dense_feature_and_full_neighbor():
-    g = graphs.random_graph(seed=9, n=200, T=3, avg_deg=4, feat_dim=12)
-    rg = graphs.ref_graph(g)
+    g = graphs.random_graph(**mg.FEAT_GRAPH)
     og = graphs.oracle_graph(g)
-    ids = np.concatenate([g["ids"][:50], [999999]]).astype(np.uint64)
-    f_ref, _ = rg.get_dense_feature(ids, 0, 12)
-    cases.eq(og.op_get_dense_feature(ids.astype(np.int64), 12), f_ref, "dense feature")
-    for et in ([0], [2, 0], [1, 1], [5]):
-        for x, y in zip(rg.get_full_neighbor(ids, et), og.get_full_neighbor(ids, et)):
-            cases.eq(y, x, "full neighbor %s" % et)
+    ids = mg.full_neighbor_ids(g)
+    cases.eq_ref(og.op_get_dense_feature(ids.astype(np.int64), mg.FEAT_GRAPH["feat_dim"]), "feat", "dense feature")
+    for i, et in enumerate(mg.FULL_NEIGHBOR_ETS):
+        for k, x in zip(("lens", "ids", "w", "t"), og.get_full_neighbor(ids, et)):
+            cases.eq_ref(x, "full%d_%s" % (i, k), "full neighbor %s: %s" % (et, k))
