@@ -68,6 +68,7 @@ SIGNATURES = {
     "eu_graph_dense_feature_dim": (_I32, [_P, _I32]),
     "eu_graph_sparse_feature_id": (_I32, [_P, C.c_char_p]),
     "eu_graph_binary_feature_id": (_I32, [_P, C.c_char_p]),
+    "eu_graph_sparse_feature_max_len": (_I64, [_P, _I32]),
     "eu_get_sparse_feature": (C.c_int, [_P, _P, _I64, _I32, _I64, _I64, _P, _P]),
     "eu_get_sparse_feature_host": (C.c_int, [_P, _P, _I64, _I32, _I64, _I64, _P, _P, _P]),
     "eu_get_binary_feature": (C.c_int, [_P, _P, _I64, _I32, _I64, _P, _P]),
@@ -96,6 +97,10 @@ SIGNATURES = {
     "eu_sample_fanout_batched": (C.c_int, [_P, _P, _I32, _I64, _P, _I32, _P, _I32, _I64, _P, _P, _P]),
     "eu_sample_fanout_host": (C.c_int, [_P, _P, _I64, _P, _I32, _P, _I32, _I64, _P, _P, _P]),
     "eu_sample_fanout_batched_host": (C.c_int, [_P, _P, _I32, _I64, _P, _I32, _P, _I32, _I64, _P, _P, _P]),
+    "eu_sample_fanout_with_feature": (C.c_int, [_P, _P, _I64, _P, _I32, _P, _I32, _I64, _P, _P, _P, _I32, _P, _P, _P, _I32, _P,
+                                                _P, _P, _P]),
+    "eu_sample_fanout_with_feature_host": (C.c_int, [_P, _P, _I64, _P, _I32, _P, _I32, _I64, _P, _P, _P, _I32, _P, _P, _P, _I32,
+                                                     _P, _P, _P, _P]),
     "eu_sage_mean_aggregate_host": (C.c_int, [_P, _P, _I64, _I32, _I32, _P]),
     "eu_sample_node": (C.c_int, [_P, _I32, _P, _I32, _P]),
     "eu_sample_node_host": (C.c_int, [_P, _I32, _P, _I32, _P]),

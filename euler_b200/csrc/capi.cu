@@ -99,6 +99,15 @@ int ctx_misc(eu_ctx* c, int64_t bytes) {
   return EU_OK;
 }
 
+int ctx_levels(eu_ctx* c, int64_t ids) {
+  if (ids <= c->levels_cap) return EU_OK;
+  if (int rc0 = refuse_growth_in_capture(c, "the fanout level scratch")) return rc0;
+  EU_CUDA(cudaStreamSynchronize(c->stream));
+  int rc = regrow(&c->d_levels, ids);
+  c->levels_cap = rc ? 0 : ids;
+  return rc;
+}
+
 int ctx_stage(eu_ctx* c, int64_t host_bytes, int64_t dev_bytes) {
   if (host_bytes > c->pin_bytes) {
     if (c->h_pin) cudaFreeHost(c->h_pin);
@@ -164,7 +173,7 @@ int eu_ctx_destroy(eu_ctx* c) {
   cudaSetDevice(c->g->device);
   cudaStreamSynchronize(c->stream);
   cudaFree(c->d_rng); cudaFree(c->d_dedup); cudaFree(c->d_first); cudaFree(c->d_rowof);
-  cudaFree(c->d_elig); cudaFree(c->d_state); cudaFree(c->d_emask); cudaFree(c->d_woff); cudaFree(c->d_blkpre); cudaFree(c->d_blkmul); cudaFree(c->d_live); cudaFree(c->d_nlive); cudaFree(c->d_front[0]); cudaFree(c->d_front[1]);
+  cudaFree(c->d_elig); cudaFree(c->d_state); cudaFree(c->d_emask); cudaFree(c->d_woff); cudaFree(c->d_blkpre); cudaFree(c->d_blkmul); cudaFree(c->d_live); cudaFree(c->d_nlive); cudaFree(c->d_front[0]); cudaFree(c->d_front[1]); cudaFree(c->d_levels);
   cudaFree(c->d_misc); cudaFree(c->d_stage); cudaFree(c->d_walkv);
   for (int i = 0; i < 2; ++i) { if (c->aux[i]) cudaStreamDestroy(c->aux[i]); if (c->ev_join[i]) cudaEventDestroy(c->ev_join[i]); }
   if (c->ev_fork) cudaEventDestroy(c->ev_fork);
@@ -217,6 +226,8 @@ int eu_ctx_reserve(eu_ctx* c, int64_t max_rows) {
   const int nb = c->n_eng;
   int rc = ctx_reserve(c, max_rows + 256 * nb, 4 * max_rows + 65 * nb);
   if (rc) return rc;
+  // eu_sample_fanout_with_feature keeps every level's engine ids: at most 2 * max_rows when every count is >= 2
+  if ((rc = ctx_levels(c, 2 * max_rows))) return rc;
   return ctx_misc(c, 256 + 4 * max_rows);
 }
 
@@ -355,6 +366,73 @@ int eu_sample_fanout_host(eu_ctx* c, const int64_t* nodes, int64_t B, const int3
                           int32_t K, const int32_t* counts, int32_t L, int64_t default_node,
                           int64_t* const* out_ids, float* const* out_w, int32_t* const* out_t) {
   return eu_sample_fanout_batched_host(c, nodes, 1, B, etypes, K, counts, L, default_node, out_ids, out_w, out_t);
+}
+
+// Host buffers for eu_sample_fanout_with_feature, sized as for the device entry point (out_sp_val[i*NS+j] holds
+// rows_i * max(1, eu_graph_sparse_feature_max_len(fid_j)) values).  Only the value prefix each out_sp_ptr covers is copied back.
+int eu_sample_fanout_with_feature_host(eu_ctx* c, const int64_t* nodes, int64_t B, const int32_t* etypes, int32_t K,
+                                       const int32_t* counts, int32_t L, int64_t default_node, int64_t* const* out_ids,
+                                       float* const* out_w, int32_t* const* out_t, int32_t ND, const int32_t* dense_fids,
+                                       const int32_t* dense_dims, float* const* out_dense, int32_t NS, const int32_t* sparse_fids,
+                                       const int64_t* sparse_defaults, int64_t* const* out_sp_ptr, int64_t* const* out_sp_val) {
+  if (!c || B < 0 || L < 0 || L > 16 || ND < 0 || NS < 0 || (L > 0 && !counts) || (B > 0 && !nodes) ||
+      (int64_t)(L + 1) * ND > kMaxFeatSegs || (int64_t)(L + 1) * NS > kMaxFeatSegs || (ND > 0 && (!dense_dims || !out_dense)) ||
+      (NS > 0 && (!sparse_fids || !out_sp_ptr || !out_sp_val))) {
+    set_error("eu_sample_fanout_with_feature_host: bad argument");
+    return EU_ERR_INVALID;
+  }
+  EU_CUDA(cudaSetDevice(c->g->device));
+  HostIO io{c};
+  int64_t rows[17];
+  rows[0] = B;
+  for (int l = 0; l < L; ++l) {
+    if (counts[l] < 0) { set_error("negative count"); return EU_ERR_INVALID; }
+    rows[l + 1] = rows[l] * counts[l];
+  }
+  const int64_t o_nodes = io.take(8 * B);
+  int64_t o_ids[16], o_w[16], o_t[16];
+  for (int l = 0; l < L; ++l) { o_ids[l] = io.take(8 * rows[l + 1]); o_w[l] = io.take(4 * rows[l + 1]); o_t[l] = io.take(4 * rows[l + 1]); }
+  std::vector<int64_t> o_dense((L + 1) * ND), o_ptr((L + 1) * NS), o_val((L + 1) * NS), ptr_last((L + 1) * NS);
+  std::vector<float*> d_dense((L + 1) * ND);
+  std::vector<int64_t*> d_ptr((L + 1) * NS), d_val((L + 1) * NS);
+  for (int i = 0; i <= L; ++i) {
+    for (int j = 0; j < ND; ++j) o_dense[i * ND + j] = io.take(4 * rows[i] * (dense_dims[j] > 0 ? dense_dims[j] : 0));
+    for (int j = 0; j < NS; ++j) {
+      o_ptr[i * NS + j] = io.take(8 * (rows[i] + 1));
+      o_val[i * NS + j] = io.take(8 * rows[i] * std::max<int64_t>(1, eu_graph_sparse_feature_max_len(c->g, sparse_fids[j])));
+    }
+  }
+  int rc = ctx_stage(c, io.st.off, io.st.off);   // always through the pinned stage: the value prefix is known only at the end
+  if (rc) return rc;
+  if ((rc = io.in(o_nodes, nodes, 8 * B))) return rc;
+  int64_t* d_ids[16]; float* d_w[16]; int32_t* d_t[16];
+  for (int l = 0; l < L; ++l) { d_ids[l] = (int64_t*)io.dev(o_ids[l]); d_w[l] = (float*)io.dev(o_w[l]); d_t[l] = (int32_t*)io.dev(o_t[l]); }
+  for (size_t k = 0; k < d_dense.size(); ++k) d_dense[k] = (float*)io.dev(o_dense[k]);
+  for (size_t k = 0; k < d_ptr.size(); ++k) { d_ptr[k] = (int64_t*)io.dev(o_ptr[k]); d_val[k] = (int64_t*)io.dev(o_val[k]); }
+  rc = eu_sample_fanout_with_feature(c, (const int64_t*)io.dev(o_nodes), B, etypes, K, counts, L, default_node, d_ids, d_w, d_t, ND,
+                                     dense_fids, dense_dims, d_dense.data(), NS, sparse_fids, sparse_defaults, d_ptr.data(), d_val.data());
+  if (rc) return rc;
+  for (int l = 0; l < L; ++l) {
+    if (out_ids && (rc = io.out(o_ids[l], out_ids[l], 8 * rows[l + 1]))) return rc;
+    if (out_w && (rc = io.out(o_w[l], out_w[l], 4 * rows[l + 1]))) return rc;
+    if (out_t && (rc = io.out(o_t[l], out_t[l], 4 * rows[l + 1]))) return rc;
+  }
+  for (int i = 0; i <= L; ++i)
+    for (int j = 0; j < ND; ++j)
+      if ((rc = io.out(o_dense[i * ND + j], out_dense[i * ND + j], 4 * rows[i] * (dense_dims[j] > 0 ? dense_dims[j] : 0)))) return rc;
+  // the pointer arrays first: they say how many values to bring back
+  for (size_t k = 0; k < o_ptr.size(); ++k) EU_CUDA(cudaMemcpyAsync((char*)c->h_pin + o_ptr[k], io.dev(o_ptr[k]), 8 * (size_t)(rows[k / NS] + 1), cudaMemcpyDeviceToHost, c->stream));
+  if ((rc = io.finish())) return rc;
+  for (size_t k = 0; k < o_ptr.size(); ++k) {
+    const int64_t n = rows[k / NS];
+    const int64_t* hp = (const int64_t*)((char*)c->h_pin + o_ptr[k]);
+    memcpy(out_sp_ptr[k], hp, 8 * (size_t)(n + 1));
+    ptr_last[k] = hp[n];
+    EU_CUDA(cudaMemcpyAsync((char*)c->h_pin + o_val[k], io.dev(o_val[k]), 8 * (size_t)ptr_last[k], cudaMemcpyDeviceToHost, c->stream));
+  }
+  EU_CUDA(cudaStreamSynchronize(c->stream));
+  for (size_t k = 0; k < o_val.size(); ++k) memcpy(out_sp_val[k], (char*)c->h_pin + o_val[k], 8 * (size_t)ptr_last[k]);
+  return EU_OK;
 }
 
 int eu_sample_neighbor_host(eu_ctx* c, const int64_t* nodes, int64_t B, const int32_t* etypes,

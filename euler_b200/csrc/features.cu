@@ -5,6 +5,8 @@
 //                                               entry {i, 0} = default_value
 //   tf_euler GetBinaryFeature                   tf_euler/kernels/get_binary_feature_op.cc          one string per node
 // Same shape as the full-neighbor listing: per-node lengths -> cub inclusive scan -> copy; no host sync in the device entry points.
+// The kernels walk a table of segments, so one length launch, one scan and one fill serve every (level, feature) of
+// eu_sample_fanout_with_feature; the single-feature entry points are the one-segment case.
 #include <cub/device/device_scan.cuh>
 
 #include <algorithm>
@@ -21,40 +23,77 @@ __device__ __forceinline__ void ragged_slice(const int64_t* __restrict__ ptr, in
   *e = ptr[row * S + fid + 1];
 }
 
-template <bool SPARSE>
-__global__ void k_ragged_len(DevGraph g, const unsigned long long* __restrict__ nodes, int64_t M, int32_t fid,
-                             long long* __restrict__ out_ptr) {
+// Segment s of a launch: rows [start, start + rows) fetch slot `fid` of ids[0 .. rows).  lens[1 + i] is the length of launch row
+// i (lens[0] = 0); after the inclusive scan, lens[i] is where row i's values begin in the launch, and segment s owns
+// out_ptr[r] = lens[start + r] - lens[start].  The one-segment entry points scan straight into their out_ptr (lens == out_ptr).
+struct RaggedSeg {
+  const unsigned long long* ids;
+  long long* out_ptr;          // [rows + 1]; written by k_ragged_fill only when the launch scans into scratch
+  long long* out_values;       // SPARSE
+  unsigned char* out_bytes;    // binary
+  int64_t start, cap;          // cap: entries of the value buffer
+  long long default_value;
+  int32_t fid;
+};
+
+template <bool SPARSE, int N>
+__global__ void k_ragged_len(DevGraph g, SegTable<RaggedSeg, N> t, long long* __restrict__ lens) {
   const int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
-  if (i == 0) out_ptr[0] = 0;
-  if (i >= M) return;
+  if (i == 0) lens[0] = 0;
+  if (i >= t.rows) return;
+  const RaggedSeg& q = t.s[seg_of(t, i)];
   int64_t b, e;
-  const int64_t row = lookup_row(g, nodes[i]);
-  if (SPARSE) ragged_slice(g.u64_ptr, g.n_u64_slots, row, fid, &b, &e);
-  else ragged_slice(g.bin_ptr, g.n_bin_slots, row, fid, &b, &e);
+  const int64_t row = lookup_row(g, q.ids[i - q.start]);
+  if (SPARSE) ragged_slice(g.u64_ptr, g.n_u64_slots, row, q.fid, &b, &e);
+  else ragged_slice(g.bin_ptr, g.n_bin_slots, row, q.fid, &b, &e);
   long long len = e - b;
   if (SPARSE && len == 0) len = 1;   // one default entry (get_sparse_feature_op.cc:96-99)
-  out_ptr[i + 1] = len;
+  lens[i + 1] = len;
 }
 
-template <bool SPARSE>
-__global__ void __launch_bounds__(256) k_ragged_fill(DevGraph g, const unsigned long long* __restrict__ nodes, int64_t M, int32_t fid,
-                                                     long long default_value, const long long* __restrict__ out_ptr, int64_t cap,
-                                                     long long* __restrict__ out_values, unsigned char* __restrict__ out_bytes) {
+template <bool SPARSE, int N>
+__global__ void __launch_bounds__(256) k_ragged_fill(DevGraph g, SegTable<RaggedSeg, N> t, const long long* __restrict__ lens,
+                                                     bool write_ptr) {
   const int lane = threadIdx.x & 31;
+  const int64_t gtid = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
   const int64_t nwarps = ((int64_t)gridDim.x * blockDim.x) >> 5;
-  for (int64_t i = (blockIdx.x * (int64_t)blockDim.x + threadIdx.x) >> 5; i < M; i += nwarps) {
+  if (write_ptr && gtid < t.n) t.s[N == 1 ? 0 : gtid].out_ptr[0] = 0;   // also for segments without rows
+  for (int64_t i = gtid >> 5; i < t.rows; i += nwarps) {
+    const RaggedSeg& q = t.s[seg_of(t, i)];
+    const int64_t r = i - q.start;
     int64_t b, e;
-    const int64_t row = lookup_row(g, nodes[i]);
-    if (SPARSE) ragged_slice(g.u64_ptr, g.n_u64_slots, row, fid, &b, &e);
-    else ragged_slice(g.bin_ptr, g.n_bin_slots, row, fid, &b, &e);
-    const int64_t o = out_ptr[i];
+    const int64_t row = lookup_row(g, q.ids[r]);
+    if (SPARSE) ragged_slice(g.u64_ptr, g.n_u64_slots, row, q.fid, &b, &e);
+    else ragged_slice(g.bin_ptr, g.n_bin_slots, row, q.fid, &b, &e);
+    const long long base = lens[q.start];
+    const int64_t o = lens[i] - base;
+    if (write_ptr && lane == 0) q.out_ptr[r + 1] = lens[i + 1] - base;
+    const int64_t cap = q.cap;
     if (SPARSE) {
-      if (e == b) { if (lane == 0 && o < cap) out_values[o] = default_value; continue; }
-      for (int64_t k = lane; k < e - b; k += 32) if (o + k < cap) out_values[o + k] = (long long)g.u64_val[b + k];
+      if (e == b) { if (lane == 0 && o < cap) q.out_values[o] = q.default_value; continue; }
+      for (int64_t k = lane; k < e - b; k += 32) if (o + k < cap) q.out_values[o + k] = (long long)g.u64_val[b + k];
     } else {
-      for (int64_t k = lane; k < e - b; k += 32) if (o + k < cap) out_bytes[o + k] = g.bin_val[b + k];
+      for (int64_t k = lane; k < e - b; k += 32) if (o + k < cap) q.out_bytes[o + k] = g.bin_val[b + k];
     }
   }
+}
+
+// length launch, one scan, fill launch.  lens: [rows + 1], the single segment's out_ptr or scratch behind the scan's temporary
+// storage in ctx_misc (write_ptr: the fill then writes every segment's out_ptr).
+template <bool SPARSE, int N>
+static int ragged_launch(eu_ctx* c, const SegTable<RaggedSeg, N>& t, long long* lens, bool write_ptr, bool fill, size_t tmp) {
+  const DevGraph& d = c->g->d;
+  cudaStream_t s = c->stream;
+  k_ragged_len<SPARSE, N><<<(unsigned)ceil_div(std::max<int64_t>(t.rows, 1), 256), 256, 0, s>>>(d, t, lens);
+  EU_LAUNCHED();
+  EU_CUDA(cub::DeviceScan::InclusiveSum(c->d_misc, tmp, lens, lens, (int)(t.rows + 1), s));
+  EU_LAUNCHED();
+  if (fill) {
+    const unsigned blocks = (unsigned)std::max<int64_t>(1, std::min<int64_t>(ceil_div(t.rows * 32, 256), 148 * 8));
+    k_ragged_fill<SPARSE, N><<<blocks, 256, 0, s>>>(d, t, lens, write_ptr);
+    EU_LAUNCHED();
+  }
+  return EU_OK;
 }
 
 template <bool SPARSE>
@@ -66,23 +105,38 @@ static int ragged_get(eu_ctx* c, const int64_t* nodes, int64_t M, int32_t fid, i
   }
   EU_CUDA(cudaSetDevice(c->g->device));
   if (M >= ((int64_t)1 << 31)) { set_error("%s: more than 2^31 nodes", what); return EU_ERR_UNSUPPORTED; }
-  const DevGraph& d = c->g->d;
-  cudaStream_t s = c->stream;
   size_t tmp = 0;
-  cub::DeviceScan::InclusiveSum((void*)nullptr, tmp, (long long*)nullptr, (long long*)nullptr, (int)(M + 1), s);
+  cub::DeviceScan::InclusiveSum((void*)nullptr, tmp, (long long*)nullptr, (long long*)nullptr, (int)(M + 1), c->stream);
   int rc = ctx_misc(c, (int64_t)tmp + 256);
   if (rc) return rc;
-  k_ragged_len<SPARSE><<<(unsigned)ceil_div(std::max<int64_t>(M, 1), 256), 256, 0, s>>>(d, (const unsigned long long*)nodes, M, fid, (long long*)out_ptr);
-  EU_LAUNCHED();
-  EU_CUDA(cub::DeviceScan::InclusiveSum(c->d_misc, tmp, (long long*)out_ptr, (long long*)out_ptr, (int)(M + 1), s));
-  EU_LAUNCHED();
-  if (cap > 0 && M > 0) {
-    const unsigned blocks = (unsigned)std::min<int64_t>(ceil_div(M * 32, 256), 148 * 8);
-    k_ragged_fill<SPARSE><<<blocks, 256, 0, s>>>(d, (const unsigned long long*)nodes, M, fid, (long long)default_value, (const long long*)out_ptr, cap,
-                                                 (long long*)out_values, out_bytes);
-    EU_LAUNCHED();
+  SegTable<RaggedSeg, 1> t{};
+  t.n = 1;
+  t.rows = M;
+  t.s[0] = RaggedSeg{(const unsigned long long*)nodes, (long long*)out_ptr, (long long*)out_values, out_bytes, 0, cap,
+                     (long long)default_value, fid};
+  return ragged_launch<SPARSE, 1>(c, t, (long long*)out_ptr, false, cap > 0 && M > 0, tmp);
+}
+
+int sparse_feature_segments(eu_ctx* c, const SparseSeg* segs, int n) {
+  if (n < 1 || n > kMaxFeatSegs) { set_error("sparse features: %d segments (1..%d)", n, kMaxFeatSegs); return EU_ERR_UNSUPPORTED; }
+  SegTable<RaggedSeg, kMaxFeatSegs> t{};
+  t.n = n;
+  for (int k = 0; k < n; ++k) {
+    const SparseSeg& a = segs[k];
+    if (a.rows < 0 || a.cap < 0 || !a.out_ptr || (a.rows > 0 && !a.ids) || (a.cap > 0 && !a.out_values)) {
+      set_error("sparse features: bad segment %d", k);
+      return EU_ERR_INVALID;
+    }
+    t.s[k] = RaggedSeg{a.ids, (long long*)a.out_ptr, (long long*)a.out_values, nullptr, t.rows, a.cap, (long long)a.default_value, a.fid};
+    t.rows += a.rows;
   }
-  return EU_OK;
+  if (t.rows >= ((int64_t)1 << 31)) { set_error("sparse features: more than 2^31 rows in all"); return EU_ERR_UNSUPPORTED; }
+  size_t tmp = 0;
+  cub::DeviceScan::InclusiveSum((void*)nullptr, tmp, (long long*)nullptr, (long long*)nullptr, (int)(t.rows + 1), c->stream);
+  const int64_t lens_off = ((int64_t)tmp + 255) & ~(int64_t)255;
+  int rc = ctx_misc(c, lens_off + 8 * (t.rows + 1));
+  if (rc) return rc;
+  return ragged_launch<true, kMaxFeatSegs>(c, t, (long long*)((char*)c->d_misc + lens_off), true, true, tmp);
 }
 
 // host buffers: lengths first (total), then the values when cap allows

@@ -420,6 +420,10 @@ int eu_graph_create(const eu_graph_desc* desc, int device, eu_graph** out) {
     TRY(upload(g, &d.u64_ptr, desc->u64_ptr, n * S + 1));
     TRY(upload(g, (const uint64_t**)&d.u64_val, desc->u64_val, desc->u64_ptr[n * S]));
     for (int64_t k = 0; k < S; ++k) g->sparse_feature_names.push_back("u64_" + std::to_string(k));
+    g->u64_max_len.assign(S, 0);
+    for (int64_t r = 0; r < n; ++r)
+      for (int64_t k = 0; k < S; ++k)
+        g->u64_max_len[k] = std::max(g->u64_max_len[k], desc->u64_ptr[r * S + k + 1] - desc->u64_ptr[r * S + k]);
   }
   if (desc->n_bin_slots > 0 && desc->bin_ptr) {
     const int64_t S = desc->n_bin_slots;
@@ -637,6 +641,10 @@ int32_t eu_graph_binary_feature_id(const eu_graph* g, const char* name) {
 int32_t eu_graph_dense_feature_dim(const eu_graph* g, int32_t fid) {
   if (!g || fid < 0 || fid >= g->d.n_slots) return -1;
   return g->d.slot_dim[fid];
+}
+int64_t eu_graph_sparse_feature_max_len(const eu_graph* g, int32_t fid) {
+  if (!g || fid < 0 || fid >= (int32_t)g->u64_max_len.size()) return 0;
+  return g->u64_max_len[fid];
 }
 int32_t eu_graph_node_type_id(const eu_graph* g, const char* name) {
   if (!g || !name) return -1;

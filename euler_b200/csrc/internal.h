@@ -64,6 +64,7 @@ struct eu_graph {
   std::vector<std::string> edge_type_names, node_type_names;
   std::vector<std::string> dense_feature_names;  // per slot, without the "dense_" prefix
   std::vector<std::string> sparse_feature_names, binary_feature_names;   // per slot, without the "sparse_" / "binary_" prefix
+  std::vector<int64_t> u64_max_len;    // per uint64 slot: the most values any node holds in it
   // edges (eu_graph_set_edges): device store, per-type alias samplers in edge_map_ order, feature names
   eu::DevEdges e{};
   bool edges_set = false;
@@ -121,6 +122,8 @@ struct eu_ctx {
   int32_t* d_live = nullptr;         // [rows] rows that sample, compacted by k_prepare
   unsigned int* d_nlive = nullptr;   // their number
   unsigned long long* d_front[2] = {nullptr, nullptr};  // engine-id frontier ping-pong [rows]
+  unsigned long long* d_levels = nullptr;  // engine ids of every hop of one fanout, back to back (eu_sample_fanout_with_feature)
+  int64_t levels_cap = 0;
   // extra scratch for walks / scatter
   void* d_misc = nullptr;
   int64_t misc_bytes = 0;
@@ -161,6 +164,7 @@ int64_t hop_scratch_rows(int nb, int64_t rows_b);
 int64_t hop_table_slots(int nb, int64_t rows_b);
 int64_t hop_table_cap(int64_t rows_b);   // dedup slots per batch (region stride = cap + 1)
 int ctx_misc(eu_ctx* c, int64_t bytes);
+int ctx_levels(eu_ctx* c, int64_t ids);   // d_levels holds at least `ids` engine ids
 int refuse_growth_in_capture(eu_ctx* c, const char* what);   // EU_ERR_STATE if the ctx stream is being captured
 int ctx_stage(eu_ctx* c, int64_t host_bytes, int64_t dev_bytes);
 int graph_build_sampler(eu_graph* g);
@@ -171,4 +175,31 @@ int hop(eu_ctx* c, const unsigned long long* seeds, int64_t rows, const int32_t*
         int32_t count, int64_t default_node, unsigned long long* eng_ids, int64_t* out_ids,
         float* out_w, int32_t* out_t, int hop_index, bool pre_inserted, bool insert_next, int nb,
         const int32_t* rows_act = nullptr, bool raw = false);
+
+// Multi-segment feature fetches: one launch set serves several (ids, output) pairs, e.g. every (level, feature) of a fanout.
+// Segment s covers rows [start_s, start_s + rows_s) of the launch; seg_of finds the segment of a row.
+constexpr int kMaxFeatSegs = 64;
+template <class Seg, int N>
+struct SegTable {
+  int32_t n;      // segments in use (<= N)
+  int64_t rows;   // total rows
+  Seg s[N];
+};
+template <class Seg, int N>
+__device__ __forceinline__ int seg_of(const SegTable<Seg, N>& t, int64_t i) {
+  if (N == 1) return 0;
+  int lo = 0, hi = t.n - 1;   // last segment with start <= i (an empty segment shares its start with the next one)
+  while (lo < hi) {
+    const int mid = (lo + hi + 1) >> 1;
+    if (t.s[mid].start <= i) lo = mid; else hi = mid - 1;
+  }
+  return lo;
+}
+struct DenseSeg { const unsigned long long* ids; int64_t rows; int32_t fid; int32_t dim; float* out; };
+// one k_feature launch for all segments (mp_ops.cu)
+int dense_feature_segments(eu_ctx* c, const DenseSeg* segs, int n);
+struct SparseSeg { const unsigned long long* ids; int64_t rows; int32_t fid; int64_t default_value; int64_t cap; int64_t* out_ptr;
+                   int64_t* out_values; };
+// three launches (lengths, one scan, fill) for all segments, no host sync (features.cu)
+int sparse_feature_segments(eu_ctx* c, const SparseSeg* segs, int n);
 }  // namespace eu

@@ -776,6 +776,40 @@ int hop(eu_ctx* c, const unsigned long long* seeds, int64_t rows_b, const int32_
   return EU_OK;
 }
 
+// The hop chain of a fanout over nb batches.  levels == null: the engine ids of hops 0..L-2 live in the ping-pong frontier only.
+// Otherwise hop l writes its engine ids, the last hop's included, to levels + (rows of hops 0..l-1): the caller keeps every
+// level's frontier (d_levels, sized by the caller).
+static int fanout_chain(eu_ctx* c, const int64_t* nodes, int32_t nb, int64_t B, const int32_t* etypes, int32_t K,
+                        const int32_t* counts, int32_t L, int64_t default_node, int64_t* const* out_ids, float* const* out_w,
+                        int32_t* const* out_t, unsigned long long* levels) {
+  // a hop with count 0 delivers nothing and neither does any hop after it: stop the chain BEFORE it, so that no hop enters
+  // ids into a dedup table that nobody would consume and wipe (the tables must be all-free when an op returns)
+  for (int l = 0; l < L; ++l)
+    if (counts[l] == 0) { L = l; break; }
+  if (B == 0) return EU_OK;
+  int64_t rows_b = B, max_rows = hop_scratch_rows(nb, B), max_slots = hop_table_slots(nb, B), widest = B * nb;
+  for (int l = 0; l < L; ++l) {
+    rows_b *= counts[l];
+    if (l + 1 < L) { max_rows = std::max(max_rows, hop_scratch_rows(nb, rows_b)); max_slots = std::max(max_slots, hop_table_slots(nb, rows_b)); }
+    widest = std::max(widest, rows_b * nb);
+  }
+  int rc = ctx_reserve(c, std::max(max_rows, widest), max_slots);
+  if (rc) return rc;
+  const unsigned long long* seeds = (const unsigned long long*)nodes;
+  rows_b = B;
+  for (int l = 0; l < L; ++l) {
+    unsigned long long* eng = levels ? levels : (l + 1 < L) ? c->d_front[l & 1] : nullptr;
+    rc = hop(c, seeds, rows_b, etypes + (int64_t)l * K, K, counts[l], default_node, eng,
+             out_ids ? out_ids[l] : nullptr, out_w ? out_w[l] : nullptr, out_t ? out_t[l] : nullptr,
+             l, /*pre_inserted=*/l > 0 && c->rng == EU_RNG_MINSTD, /*insert_next=*/l + 1 < L, nb);
+    if (rc) return rc;
+    seeds = eng;
+    rows_b *= counts[l];
+    if (levels) levels += rows_b * nb;
+  }
+  return EU_OK;
+}
+
 }  // namespace eu
 
 using namespace eu;
@@ -811,37 +845,66 @@ int eu_sample_fanout_batched(eu_ctx* c, const int64_t* nodes, int32_t nb, int64_
   if (nb > c->n_eng) { set_error("eu_sample_fanout_batched: %d batches but the ctx has %d engines (eu_ctx_set_engines)", nb, c->n_eng); return EU_ERR_INVALID; }
   for (int l = 0; l < L; ++l)
     if (counts[l] < 0) { set_error("negative count"); return EU_ERR_INVALID; }
-  // a hop with count 0 delivers nothing and neither does any hop after it: stop the chain BEFORE it, so that no hop enters
-  // ids into a dedup table that nobody would consume and wipe (the tables must be all-free when an op returns)
-  for (int l = 0; l < L; ++l)
-    if (counts[l] == 0) { L = l; break; }
-  if (B == 0) return EU_OK;
-  int64_t rows_b = B, max_rows = hop_scratch_rows(nb, B), max_slots = hop_table_slots(nb, B), widest = B * nb;
-  for (int l = 0; l < L; ++l) {
-    rows_b *= counts[l];
-    if (l + 1 < L) { max_rows = std::max(max_rows, hop_scratch_rows(nb, rows_b)); max_slots = std::max(max_slots, hop_table_slots(nb, rows_b)); }
-    widest = std::max(widest, rows_b * nb);
-  }
-  int rc = ctx_reserve(c, std::max(max_rows, widest), max_slots);
-  if (rc) return rc;
-  const unsigned long long* seeds = (const unsigned long long*)nodes;
-  rows_b = B;
-  for (int l = 0; l < L; ++l) {
-    unsigned long long* eng = (l + 1 < L) ? c->d_front[l & 1] : nullptr;
-    rc = hop(c, seeds, rows_b, etypes + (int64_t)l * K, K, counts[l], default_node, eng,
-             out_ids ? out_ids[l] : nullptr, out_w ? out_w[l] : nullptr, out_t ? out_t[l] : nullptr,
-             l, /*pre_inserted=*/l > 0 && c->rng == EU_RNG_MINSTD, /*insert_next=*/l + 1 < L, nb);
-    if (rc) return rc;
-    seeds = eng;
-    rows_b *= counts[l];
-  }
-  return EU_OK;
+  return fanout_chain(c, nodes, nb, B, etypes, K, counts, L, default_node, out_ids, out_w, out_t, nullptr);
 }
 
 int eu_sample_fanout(eu_ctx* c, const int64_t* nodes, int64_t B, const int32_t* etypes, int32_t K,
                      const int32_t* counts, int32_t L, int64_t default_node, int64_t* const* out_ids,
                      float* const* out_w, int32_t* const* out_t) {
   return eu_sample_fanout_batched(c, nodes, 1, B, etypes, K, counts, L, default_node, out_ids, out_w, out_t);
+}
+
+// tf_euler.sample_fanout_with_feature (tf_euler/kernels/sample_fanout_with_feature_op.cc): the sample_fanout chain (:59-64), then
+// the features of every level's ENGINE ids (v_select(nb_i), :65-68).  Level 0 is `nodes` as given; a default-filled slot of a
+// later level has no node (engine id 0), so it gets zeros and the sparse default whatever default_node is.
+int eu_sample_fanout_with_feature(eu_ctx* c, const int64_t* nodes, int64_t B, const int32_t* etypes, int32_t K,
+                                  const int32_t* counts, int32_t L, int64_t default_node, int64_t* const* out_ids,
+                                  float* const* out_w, int32_t* const* out_t, int32_t ND, const int32_t* dense_fids,
+                                  const int32_t* dense_dims, float* const* out_dense, int32_t NS, const int32_t* sparse_fids,
+                                  const int64_t* sparse_defaults, int64_t* const* out_sp_ptr, int64_t* const* out_sp_val) {
+  if (!c || B < 0 || L < 0 || L > 16 || ND < 0 || NS < 0 || (L > 0 && !counts) || (K > 0 && !etypes) || (B > 0 && !nodes) ||
+      (ND > 0 && (!dense_fids || !dense_dims || !out_dense)) ||
+      (NS > 0 && (!sparse_fids || !sparse_defaults || !out_sp_ptr || !out_sp_val))) {
+    set_error("eu_sample_fanout_with_feature: bad argument");
+    return EU_ERR_INVALID;
+  }
+  if ((int64_t)(L + 1) * ND > kMaxFeatSegs || (int64_t)(L + 1) * NS > kMaxFeatSegs) {
+    set_error("eu_sample_fanout_with_feature: (L+1)*ND = %d and (L+1)*NS = %d, at most %d each", (L + 1) * ND, (L + 1) * NS, kMaxFeatSegs);
+    return EU_ERR_UNSUPPORTED;
+  }
+  for (int l = 0; l < L; ++l)
+    if (counts[l] < 0) { set_error("negative count"); return EU_ERR_INVALID; }
+  for (int j = 0; j < ND; ++j)
+    if (dense_dims[j] < 0) { set_error("negative dense dimension"); return EU_ERR_INVALID; }
+  EU_CUDA(cudaSetDevice(c->g->device));
+  int64_t rows[17];
+  rows[0] = B;
+  for (int l = 0; l < L; ++l) rows[l + 1] = rows[l] * counts[l];
+  int64_t level_ids = 0;
+  for (int l = 1; l <= L; ++l) level_ids += rows[l];
+  int rc = ctx_levels(c, level_ids);
+  if (rc) return rc;
+  rc = fanout_chain(c, nodes, 1, B, etypes, K, counts, L, default_node, out_ids, out_w, out_t, c->d_levels);
+  if (rc) return rc;
+  const unsigned long long* lv[17];
+  lv[0] = (const unsigned long long*)nodes;
+  for (int l = 1; l <= L; ++l) lv[l] = l == 1 ? c->d_levels : lv[l - 1] + rows[l - 1];
+  if (ND > 0) {
+    DenseSeg segs[kMaxFeatSegs];
+    for (int i = 0; i <= L; ++i)
+      for (int j = 0; j < ND; ++j) segs[i * ND + j] = DenseSeg{lv[i], rows[i], dense_fids[j], dense_dims[j], out_dense[i * ND + j]};
+    if ((rc = dense_feature_segments(c, segs, (L + 1) * ND))) return rc;
+  }
+  if (NS > 0) {
+    SparseSeg segs[kMaxFeatSegs];
+    for (int i = 0; i <= L; ++i)
+      for (int j = 0; j < NS; ++j) {
+        const int64_t cap = rows[i] * std::max<int64_t>(1, eu_graph_sparse_feature_max_len(c->g, sparse_fids[j]));
+        segs[i * NS + j] = SparseSeg{lv[i], rows[i], sparse_fids[j], sparse_defaults[j], cap, out_sp_ptr[i * NS + j], out_sp_val[i * NS + j]};
+      }
+    if ((rc = sparse_feature_segments(c, segs, (L + 1) * NS))) return rc;
+  }
+  return EU_OK;
 }
 
 int eu_sample_node(eu_ctx* c, int32_t count, const int32_t* types, int32_t n_types, int64_t* out) {

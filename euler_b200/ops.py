@@ -171,6 +171,61 @@ def sample_fanout(nodes, edge_types, counts, default_node=-1):
     return [nodes] + ids, ws, ts
 
 
+def sample_fanout_with_feature(nodes, edge_types, count, default_node, dense_feature_names, dense_dimensions,
+                               sparse_feature_names, sparse_default_values):
+    """neighbor_ops.sample_fanout_with_feature (neighbor_ops.py:49-69; kernel sample_fanout_with_feature_op.cc).  sample_fanout
+    (same draws) plus the features of every level: level 0 is `nodes`, level l the ids hop l drew, where a default-filled slot
+    has no node and gets zeros / the sparse default whatever default_node is.  Returns (neighbors[L+1], weights[L], types[L],
+    dense[(L+1)*ND], sparse[(L+1)*NS]), features level-major (level i, feature j at i*ND + j); each sparse entry is
+    (indices i64[nnz, 2], values i64[nnz], dense_shape) as get_sparse_feature returns.  Names are looked up as "dense_"+name /
+    "sparse_"+name; ints are slot ids."""
+    nodes = _t(nodes, torch.int64).reshape(-1)
+    L = len(count)
+    ets = [get_edge_type_id(e) for e in edge_types]
+    if len(ets) != L or any(len(e) != len(ets[0]) for e in ets):
+        raise EulerError("sample_fanout_with_feature: edge_types must hold one equal-length type list per hop")
+    if len(dense_feature_names) != len(dense_dimensions) or len(sparse_feature_names) != len(sparse_default_values):
+        raise EulerError("sample_fanout_with_feature: one dimension per dense feature and one default per sparse feature")
+    g, lib = get_graph(), _lib.load()
+    et = np.ascontiguousarray(np.stack(ets) if L else np.zeros((0, 0)), dtype=np.int32)
+    cs = np.ascontiguousarray(count, dtype=np.int32)
+    dfid = np.asarray([n if isinstance(n, (int, np.integer)) else g.dense_feature_id(n) for n in dense_feature_names], np.int32)
+    ddim = np.asarray([int(d) for d in dense_dimensions], np.int32)
+    sfid = np.asarray([n if isinstance(n, (int, np.integer)) else g.sparse_feature_id(n) for n in sparse_feature_names], np.int32)
+    sdef = np.asarray([int(v) for v in sparse_default_values], np.int64)
+    dev = nodes.device
+    rows = [nodes.numel()]
+    for c in count:
+        rows.append(rows[-1] * int(c))
+    ids = [torch.empty(r, dtype=torch.int64, device=dev) for r in rows[1:]]
+    ws = [torch.empty(r, dtype=torch.float32, device=dev) for r in rows[1:]]
+    ts = [torch.empty(r, dtype=torch.int32, device=dev) for r in rows[1:]]
+    dense = [torch.empty((r, int(d)), dtype=torch.float32, device=dev) for r in rows for d in ddim]
+    maxlen = [max(1, lib.eu_graph_sparse_feature_max_len(g._h, int(f))) for f in sfid]
+    sp_ptr = [torch.empty(r + 1, dtype=torch.int64, device=dev) for r in rows for _ in sfid]
+    sp_val = [torch.empty(r * m, dtype=torch.int64, device=dev) for r in rows for m in maxlen]
+
+    def P(ts_):
+        return (C.c_void_p * max(len(ts_), 1))(*[x.data_ptr() for x in ts_])
+    ctx = _ctx_on_stream()
+    check(lib.eu_sample_fanout_with_feature(ctx._h, nodes.data_ptr(), rows[0], et.ctypes.data, et.shape[1] if L else 0,
+                                            cs.ctypes.data, L, int(default_node), P(ids), P(ws), P(ts), len(dfid),
+                                            dfid.ctypes.data, ddim.ctypes.data, P(dense), len(sfid), sfid.ctypes.data,
+                                            sdef.ctypes.data, P(sp_ptr), P(sp_val)))
+    sparse = []
+    if sp_ptr:
+        lens = [p[1:] - p[:-1] for p in sp_ptr]
+        zero = torch.zeros(1, dtype=torch.int64, device=dev)
+        # the one host sync: value counts (to cut the value arrays) and row maxima (dense_shape) of every feature
+        sizes = torch.stack([torch.cat([p[-1:], n.max().reshape(1) if n.numel() else zero]) for p, n in zip(sp_ptr, lens)]).cpu().tolist()
+        for indptr, vals, ln, (total, width) in zip(sp_ptr, sp_val, lens, sizes):
+            n = ln.numel()
+            r = torch.repeat_interleave(torch.arange(n, device=dev), ln, output_size=total)
+            cols = torch.arange(total, device=dev) - indptr[:-1][r]
+            sparse.append((torch.stack([r, cols], dim=1), vals[:total], (n, width)))
+    return [nodes] + ids, ws, ts, dense, sparse
+
+
 def sample_fanout_batched(nodes, edge_types, counts, default_node=-1, ctx=None):
     """nb independent sample_fanout calls in one set of kernel launches.  nodes: [nb, B]; batch b runs on engine b
     of `ctx` (Context.set_engines), i.e. it returns exactly what sample_fanout(nodes[b]) returns on a context

@@ -169,6 +169,9 @@ int32_t eu_graph_dense_feature_dim(const eu_graph* g, int32_t fid);
 /* slots of the uint64 ("sparse_"+name, get_sparse_feature_op.cc:75) and binary ("binary_"+name) features; -1 if unknown */
 int32_t eu_graph_sparse_feature_id(const eu_graph* g, const char* name);
 int32_t eu_graph_binary_feature_id(const eu_graph* g, const char* name);
+/* the most uint64 values any node holds in slot `fid` (computed at upload); 0 for an unknown slot.  Sizes the value buffers
+ * of eu_sample_fanout_with_feature without a lengths-first call. */
+int64_t eu_graph_sparse_feature_max_len(const eu_graph* g, int32_t fid);
 
 /* ------------------------------------------------------------------ contexts ----------------- */
 /* stream: a cudaStream_t (NULL = legacy default stream). */
@@ -180,7 +183,9 @@ int eu_ctx_seed(eu_ctx* c, uint64_t seed);           /* engine e <- seed + e; st
  * its own dedup scope), i.e. each batch is exactly one reference op call on one client thread; batching only
  * shares kernel launches.  seeds == NULL: engine e <- seed + e.  Plain ops use engine 0. */
 int eu_ctx_set_engines(eu_ctx* c, int32_t n, const uint64_t* seeds);
-int eu_ctx_reserve(eu_ctx* c, int64_t max_rows);      /* pre-size scratch (required before graph capture) */
+/* pre-size scratch (required before graph capture) for hops of up to max_rows rows; it also covers the level scratch of an
+ * eu_sample_fanout_with_feature whose levels 1..L hold at most 2 * max_rows ids in all (every count >= 2) */
+int eu_ctx_reserve(eu_ctx* c, int64_t max_rows);
 int eu_ctx_sync(eu_ctx* c);
 /* number of uniforms the MINSTD engine has produced since the last seed (synchronises) */
 int eu_ctx_draws(eu_ctx* c, uint64_t* draws);
@@ -222,6 +227,30 @@ int eu_sample_fanout_host(eu_ctx* c, const int64_t* nodes, int64_t B, const int3
 int eu_sample_fanout_batched_host(eu_ctx* c, const int64_t* nodes, int32_t nb, int64_t B, const int32_t* etypes,
                                   int32_t K, const int32_t* counts, int32_t L, int64_t default_node,
                                   int64_t* const* out_ids, float* const* out_w, int32_t* const* out_t);
+/* tf_euler.sample_fanout_with_feature -- TF op SampleFanoutWithFeature (tf_euler/python/euler_ops/neighbor_ops.py:49-69, kernel
+ * tf_euler/kernels/sample_fanout_with_feature_op.cc:95-274): eu_sample_fanout (same draws, ids, weights and types bit for bit,
+ * L <= 16) plus the dense and uint64 features of every level.  Level 0 is `nodes` as given; level l >= 1 is hop l's ENGINE ids
+ * (v_select(nb_l), :65-68), so a default-filled slot gets zeros and the sparse default whatever default_node is.  Rows of level
+ * i: rows_0 = B, rows_i = rows_{i-1} * counts[i-1]; a hop with count 0 ends the chain (later levels have 0 rows).
+ *   dense_fids / dense_dims i32[ND] (host; slot ids as eu_get_dense_feature, -1 = unknown = zeros);
+ *   out_dense[i*ND + j] -> f32[rows_i, dense_dims[j]], zero fill; a stored width above dense_dims[j] is clipped to it
+ *   (:220-237 copies the whole stored row, past the row's end).
+ *   sparse_fids i32[NS], sparse_defaults i64[NS] (host; slot ids as eu_get_sparse_feature);
+ *   out_sp_ptr[i*NS + j] -> i64[rows_i + 1] and out_sp_val[i*NS + j] -> i64[rows_i * max(1, eu_graph_sparse_feature_max_len(fid_j))]:
+ *   eu_get_sparse_feature's CSR form, a row without values owns one entry = the default (:238-257).
+ * (L+1)*ND and (L+1)*NS are at most 64 each (EU_ERR_UNSUPPORTED beyond).  One dense launch and three sparse launches serve all
+ * levels and features; no host synchronisation. */
+int eu_sample_fanout_with_feature(eu_ctx* c, const int64_t* nodes, int64_t B, const int32_t* etypes, int32_t K,
+                                  const int32_t* counts, int32_t L, int64_t default_node, int64_t* const* out_ids,
+                                  float* const* out_w, int32_t* const* out_t, int32_t ND, const int32_t* dense_fids,
+                                  const int32_t* dense_dims, float* const* out_dense, int32_t NS, const int32_t* sparse_fids,
+                                  const int64_t* sparse_defaults, int64_t* const* out_sp_ptr, int64_t* const* out_sp_val);
+/* host buffers, same sizing; out_sp_val[k] receives out_sp_ptr[k][rows] values */
+int eu_sample_fanout_with_feature_host(eu_ctx* c, const int64_t* nodes, int64_t B, const int32_t* etypes, int32_t K,
+                                       const int32_t* counts, int32_t L, int64_t default_node, int64_t* const* out_ids,
+                                       float* const* out_w, int32_t* const* out_t, int32_t ND, const int32_t* dense_fids,
+                                       const int32_t* dense_dims, float* const* out_dense, int32_t NS, const int32_t* sparse_fids,
+                                       const int64_t* sparse_defaults, int64_t* const* out_sp_ptr, int64_t* const* out_sp_val);
 /* tf_euler.sample_node -- TF op SampleNode (tf_euler/ops/sample_ops.cc:22-37, kernel
  * tf_euler/kernels/sample_node_op.cc:39-96; euler::SampleNode api.cc:32-37).  types i32[n_types]
  * (host); a single -1 means all types.  out i64[count]. */
